@@ -2,7 +2,7 @@
 """bench.py — LP relaxations solved per second on BASELINE.json configs[1]:
 a batch of 4096 independent random dense LP relaxations, m=64, n=128, float64, per GPU (weak scaling).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   (N>1: python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...)
 
 One "step" = one pass of the hot path (gm_simplex_batch_device: the simplex wave kernel) over one batch.
@@ -134,6 +134,14 @@ def make_batch(rank: int, count: int = BATCH):
     from problems import feasible_bounded_lp
     rng = np.random.default_rng(SEED + rank)
     return feasible_bounded_lp(rng, M, N, count)
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes each output array of the last timed step as out_dir/<name>.npy in float64 (the integer outputs are
+    small indices and counters, exact in float64), so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def cpu_baseline(count: int, threads: int):
@@ -280,8 +288,10 @@ def run_reference(args, rank: int, world: int):
     per_step = int(min(BATCH, max(8 * cores, rate * 200.0 / max(1, args.steps))))
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle.simplex_batch(c[:per_step], A[:per_step], b[:per_step], threads=cores)
+        o = oracle.simplex_batch(c[:per_step], A[:per_step], b[:per_step], threads=cores)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: o[k] for k in ("status", "optF", "x", "basis")})
     value = per_step * args.steps / dt
     sample = (f"the first {per_step} of the batch's {BATCH} LPs per step, {cores} threads, one LP per thread"
               if per_step < BATCH else f"the whole {BATCH}-LP batch per step, {cores} threads, one LP per thread")
@@ -357,6 +367,9 @@ def run_ours(args, rank: int, world: int, local_rank: int):
     pivots = int(stats[:, 0].sum() + stats[:, 1].sum())
     inversions = int(stats[:, 3].sum())
     assert (status == 0).all(), "bench workload must solve to optimality"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"status": status, "optF": d_optF.cpu().numpy(), "x": d_x.cpu().numpy(),
+                                         "basis": d_basis.cpu().numpy(), "stats": stats})
 
     # ---- e2e: host buffers through the C ABI, copies inside the timed region --------------------
     # results land in pinned host memory too (a device->host copy into pageable memory is staged and ~4x slower)
@@ -488,7 +501,12 @@ def main():
                     help="e2e through one launch per slice instead of one launch gated on arrival counters: required "
                          "under ncu, whose kernel replay serialises launches (a kernel that waits for a copy issued "
                          "after it would never see it)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the arrays the last step returned (rank 0's; with --impl "
+                         "reference, those of the batch prefix it solves) as DIR/<name>.npy in float64")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -498,7 +516,8 @@ def main():
                "--master-addr", "127.0.0.1", "--master-port", os.environ.get("MASTER_PORT", "29533"),
                os.path.abspath(__file__), "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup",
                str(args.warmup), "--impl", args.impl] + (["--quick"] if args.quick else []) + \
-              (["--no-streamed"] if args.no_streamed else [])
+              (["--no-streamed"] if args.no_streamed else []) + \
+              (["--dump-outputs", os.path.abspath(args.dump_outputs)] if args.dump_outputs else [])
         sys.exit(subprocess.call(cmd))
     if args.impl == "reference":
         run_reference(args, rank, world)
