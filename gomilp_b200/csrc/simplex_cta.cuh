@@ -2918,10 +2918,15 @@ struct SolverT {
                 }
                 bool again = false;
                 if constexpr (WARM) {
+                    // a cap the caller set (gm_options.max_pivots > 0) bounds the pivots of all passes together
+                    const int user_cap = P.max_pivots > 0 ? P.max_pivots : INT_MAX;
+                    const long long fresh_cap = (long long)piv1 + piv2 + 50 * (m + n) + 1000;
+                    const int retry_cap = fresh_cap < user_cap ? (int)fresh_cap : user_cap;
+                    const bool cap_left = piv1 + piv2 < user_cap;
                     if (P.robust && !P.initial_basic && !(attempt == 0 && warm)) {
-                        if (attempt == 0 && robust_retryable(status)) {
+                        if (attempt == 0 && robust_retryable(status) && cap_left) {
                             scan_fb |= 2;  // reported in stats[5], bit 1
-                            max_pivots = piv1 + piv2 + 50 * (m + n) + 1000;
+                            max_pivots = retry_cap;
                             fresh = true; warm = false; ran_main = false;
                             attempt = 1;
                             again = true;
@@ -2934,9 +2939,9 @@ struct SolverT {
                                 again = true;
                             }
                         }
-                        if (!again && attempt >= 1 && robust_retryable(status) && eps_rel < 1e-4) {
+                        if (!again && attempt >= 1 && robust_retryable(status) && eps_rel < 1e-4 && cap_left) {
                             eps_rel *= 100.0;  // still stuck: once more from scratch with a coarser perturbation
-                            max_pivots = piv1 + piv2 + 50 * (m + n) + 1000;
+                            max_pivots = retry_cap;
                             fresh = true; warm = false; ran_main = false;
                             attempt = 1;
                             again = true;

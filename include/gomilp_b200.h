@@ -52,7 +52,9 @@ int gm_last_timing(gm_timing* out);
 
 /* Engine knobs with reference-compatible defaults (0 / negative = default). */
 typedef struct gm_options {
-    int32_t max_pivots;      /* safety cap per LP; the reference has none. default 50*(m+n)+1000 */
+    int32_t max_pivots;      /* safety cap per LP; the reference has none. default 50*(m+n)+1000. A cap set here bounds
+                                the pivots of all passes of an LP together, robust passes included: an LP that reaches
+                                it returns GM_ERR_ITERATION_LIMIT. Only the default cap is raised by the robust passes. */
     int32_t refactor_period; /* pivots between rebuilds of the basis inverse. default 100 */
     int32_t force_tier;      /* 0 auto, else the gm_timing.tier to force (GM_ERR_TOO_LARGE if it does not fit) */
     int32_t reserved;        /* 1: tier 4 without the TMA staging ring (plain loads), for A/B measurements */

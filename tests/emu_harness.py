@@ -88,7 +88,8 @@ def simplex_batch(c, A, b, tol=0.0, bvar=None, bsign=None, brhs=None, initial_ba
 
 
 def coop_batch(c, A, b, tol=0.0, bvar=None, bsign=None, brhs=None, T=64, G=3, groups=1, max_pivots=0,
-               refactor_period=0, shared_root=False, shuffle_order=False, trace_cap=0, trace_lp=0, smem_panel=True):
+               refactor_period=0, shared_root=False, shuffle_order=False, trace_cap=0, trace_lp=0, smem_panel=True,
+               initial_basic=None):
     """Batch of LPs through the emulated COOPERATIVE tier: `groups` groups of G CTAs (T threads each) share the work."""
     A = np.ascontiguousarray(A, dtype=np.float64)
     c = np.ascontiguousarray(c, dtype=np.float64)
@@ -112,9 +113,10 @@ def coop_batch(c, A, b, tol=0.0, bvar=None, bsign=None, brhs=None, T=64, G=3, gr
     basis = np.zeros((count, m), dtype=np.int64)
     stats = np.zeros((count, 8), dtype=np.int32)
     trace = np.full((max(trace_cap, 1), 4), -1, dtype=np.int32)
+    ib = None if initial_basic is None else np.ascontiguousarray(initial_basic, dtype=np.int64).reshape(count, m)
     lib().emu_set_coop_pan(C.c_int(int(smem_panel)))
     rc = lib().emu_coop_batch(C.c_int(count), _p(c), _p(A), _p(b), C.c_longlong(cs), C.c_longlong(As), C.c_longlong(bs),
-                              C.c_int(n0), C.c_int(m0), C.c_int(n0), C.c_int(L), _p(bvar), _p(bsign), _p(brhs), None,
+                              C.c_int(n0), C.c_int(m0), C.c_int(n0), C.c_int(L), _p(bvar), _p(bsign), _p(brhs), _p(ib),
                               C.c_double(tol), C.c_int(max_pivots), C.c_int(refactor_period), _p(status), _p(optF),
                               _p(x), C.c_longlong(x_len), C.c_int(x_len), _p(basis), _p(stats), C.c_int(T), C.c_int(G),
                               C.c_int(groups), C.c_int(int(shuffle_order)), _p(trace) if trace_cap else None,
