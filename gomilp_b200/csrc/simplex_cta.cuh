@@ -524,14 +524,21 @@ struct SolverT {
     }
 
     // ---- verifyInputs, simplex.go:385-439 ---------------------------------------------------------
+    // The REG tier reads A from HBM once: straight into W (which keeps the original column order there), and the
+    // tests below read W. The other tiers read A0 where it lies.
     GM_DEV int verify_inputs() {
         const int t = gm_tid(), T = gm_nthreads();
         const int warp = t >> 5, lane = t & 31, nw = T >> 5;
+        if constexpr (REG) load_w_reg();
+        auto a0 = [&](int i, int j) -> double {
+            if constexpr (REG) return W[i * ldw + j];
+            else return gm_ldg(A0 + (size_t)i * lda + j);
+        };
         // first all-zero row (only root rows can be: a branch row always holds its slack's 1)
         int zr = INT_MAX;
         for (int i = warp; i < m0; i += nw) {
             int nz = 0;
-            for (int j = lane; j < n0; j += 32) nz |= (gm_ldg(A0 + (size_t)i * lda + j) != 0.0);
+            for (int j = lane; j < n0; j += 32) nz |= (a0(i, j) != 0.0);
             nz = gm_any(nz);
             if (!nz && i < zr) zr = i;
         }
@@ -541,13 +548,33 @@ struct SolverT {
         int zc = INT_MAX;
         for (int j = t; j < n0; j += T) {
             int nz = 0;
-            for (int i = 0; i < m0 && !nz; ++i) nz = (gm_ldg(A0 + (size_t)i * lda + j) != 0.0);
+            for (int i = 0; i < m0 && !nz; ++i) nz = (a0(i, j) != 0.0);
             for (int k = 0; k < L && !nz; ++k) nz = (bvar[k] == j && bsign[k] != 0.0);
             if (!nz && j < zc) zc = j;
         }
         zc = block_min_int(T, [&](int k) { return k == t ? zc : INT_MAX; });
         if (zc != INT_MAX) return src_c(zc) < 0.0 ? GM_ERR_UNBOUNDED : GM_ERR_ZERO_COLUMN;
         return GM_OK;
+    }
+
+    // REG tier: W[i][v] = [A0 0; G I][i][v] for v < n, zero rows from m up to wrows. A thread owns one column and
+    // eight rows at a time, with the eight loads issued before the stores. Ends with a barrier.
+    GM_DEV void load_w_reg() {
+        const int t = gm_tid(), T = gm_nthreads();
+        int S = pow2ceil(n);
+        if (S > T) S = T;
+        const int RGn = T / S, col = t % S, rg = t / S;
+        for (int v = col; v < n; v += S) {
+            for (int i0 = rg * 8; i0 < wrows; i0 += RGn * 8) {
+                double w8[8];
+#pragma unroll
+                for (int u = 0; u < 8; ++u) w8[u] = i0 + u < m ? src_a(i0 + u, v) : 0.0;
+#pragma unroll
+                for (int u = 0; u < 8; ++u) W[(i0 + u) * ldw + v] = w8[u];
+            }
+        }
+        w_loaded = true;
+        gm_sync();
     }
 
     // ---- W / cost vectors for the current basis (extractColumns :474-488, nonBasicIdx :174-197) -----
@@ -581,10 +608,7 @@ struct SolverT {
             }
         }
         if constexpr (REG) {
-            if (!w_loaded) {
-                for_each_2d(wrows, n, [&](int i, int v) { W[i * ldw + v] = i < m ? src_a(i, v) : 0.0; });
-                w_loaded = true;
-            }
+            if (!w_loaded) load_w_reg();  // scan_basis used W as scratch
             if (phase1)
                 for (int i = t; i < wrows; i += T) W[i * ldw + n] = i < m ? art[i] : 0.0;
         } else {
@@ -665,14 +689,6 @@ struct SolverT {
     // Basis-inverse storage. Generic tiers: Bi is an m x ldb array (shared memory or HBM). REG tier:
     // registers, with the Bi slot of the workspace used as a 64 x 68 staging tile.
     // =================================================================================================
-    GM_DEV double reg_sel(int jj) const {
-        double v = 0.0;
-#pragma unroll
-        for (int u = 0; u < (REG ? 16 : 1); ++u)
-            if (u == jj) v = breg[u];
-        return v;
-    }
-
     GM_DEV void reg_dump() {  // staging tile <- registers (ends with a barrier)
         const int t = gm_tid(), row = t >> 2, q = t & 3;
 #pragma unroll
@@ -826,6 +842,21 @@ struct SolverT {
         return 0;
     }
 
+    // sum_{i < m} |M[i * ld]| in ascending i: eight loads are issued ahead of their (still sequential) adds
+    GM_DEV double col_abs_sum(const double* M, int ld) const {
+        double s = 0;
+        int i = 0;
+        for (; i + 8 <= m; i += 8) {
+            double v[8];
+#pragma unroll
+            for (int u = 0; u < 8; ++u) v[u] = M[(i + u) * ld];
+#pragma unroll
+            for (int u = 0; u < 8; ++u) s += fabs(v[u]);
+        }
+        for (; i < m; ++i) s += fabs(M[i * ld]);
+        return s;
+    }
+
     // The same Gauss-Jordan inversion with the matrix in registers: two barriers per elimination step,
     // pivot row and displaced row exchanged through prow / t1, column interchanges undone in one pass
     // through the staging tile.
@@ -841,70 +872,19 @@ struct SolverT {
         rs += gm_shfl_xor(rs, 2);
         if (row >= m) rs = 0.0;
         const double anorm_inf = block_max(T, [&](int k) { return k == t ? rs : 0.0; });
-        const double anorm_1 = block_max(m, [&](int j) {
-            double s = 0;
-            const int cj = basic[j];
-            for (int i = 0; i < m; ++i) s += fabs(W[i * ldw + cj]);
-            return s;
-        });
+        const double anorm_1 = block_max(m, [&](int j) { return col_abs_sum(W + basic[j], ldw); });
+        // Steps k = 4 jj + kq, kq = 0..3, work on columns 4 jj + q, which a rotation of the registers after every
+        // fourth step keeps in breg[0], so that every register index is a constant. prow / t1 carry their rows in the
+        // same rotated order. Sixteen rotations restore the natural order, also after a singular pivot.
         int singular = 0;
-        for (int k = 0; k < m; ++k) {
-            const int kq = k & 3;
-            const double sel = reg_sel(k >> 2);
-            double key = (q == kq && row >= k && row < m) ? fabs(sel) : -1.0;
-            if (key != key) key = INFINITY;
-            // Idamax: first largest |.| in column k at or below the diagonal (dgetf2.go:43-45). The bit
-            // pattern of a non-negative double is monotone, so two unsigned REDUX.MAX give the maximum
-            // and a REDUX.MIN over the rows that hold it gives the first one. key = -1 marks "not a candidate".
-            unsigned long long kb = key >= 0.0 ? gm_d2bits(key) : 0ull;
-            unsigned hi = (unsigned)(kb >> 32), lo = (unsigned)kb;
-            unsigned mh = gm_warp_max_u32(hi);
-            unsigned ml = gm_warp_max_u32(hi == mh ? lo : 0u);
-            int idx = gm_warp_min_int((key >= 0.0 && hi == mh && lo == ml) ? row : INT_MAX);
-            if (lane == 0) { redi[warp] = (int)mh; redi[32 + warp] = (int)ml; redi[64 + warp] = idx; }
-            gm_sync();
-            hi = (unsigned)redi[lane & (nw - 1)];
-            lo = (unsigned)redi[32 + (lane & (nw - 1))];
-            idx = redi[64 + (lane & (nw - 1))];
-            mh = gm_warp_max_u32(hi);
-            ml = gm_warp_max_u32(hi == mh ? lo : 0u);
-            idx = gm_warp_min_int((hi == mh && lo == ml) ? idx : INT_MAX);
-            key = idx == INT_MAX ? -1.0 : gm_bits2d(((unsigned long long)mh << 32) | ml);
-            if (!(key > 0.0) || key == INFINITY) { singular = 1; break; }
-            const int p = idx;
-            double f = gm_shfl_idx(sel, (lane & ~3) | kq);  // my row's entry in column k
-            if (row == p) {
-                const double inv = 1.0 / f;
+#pragma unroll 1
+        for (int jj = 0; jj < 16; ++jj) {
+#pragma unroll 1
+            for (int kq = 0; kq < 4 && 4 * jj + kq < m && !singular; ++kq) singular = eliminate_reg(4 * jj + kq, kq);
+            const double b0 = breg[0];
 #pragma unroll
-                for (int jj = 0; jj < (REG ? 16 : 1); ++jj) {
-                    const int col = 4 * jj + q;
-                    prow[col] = (col == k ? 1.0 : breg[jj]) * inv;
-                }
-            }
-            if (row == k && p != k) {
-#pragma unroll
-                for (int jj = 0; jj < (REG ? 16 : 1); ++jj) t1[4 * jj + q] = breg[jj];
-            }
-            if (t == 0) ipiv[k] = p;
-            gm_sync();
-            if (row == k) {
-#pragma unroll
-                for (int jj = 0; jj < (REG ? 16 : 1); ++jj) breg[jj] = prow[4 * jj + q];
-            } else {
-                if (row == p) {  // adopt the displaced row k
-#pragma unroll
-                    for (int jj = 0; jj < (REG ? 16 : 1); ++jj) breg[jj] = t1[4 * jj + q];
-                    f = t1[k];
-                }
-                if (f != 0.0) {
-#pragma unroll
-                    for (int jj = 0; jj < (REG ? 16 : 1); ++jj) {
-                        const int col = 4 * jj + q;
-                        const double base = (col == k) ? 0.0 : breg[jj];
-                        breg[jj] = base - f * prow[col];
-                    }
-                }
-            }
+            for (int u = 0; u < (REG ? 15 : 0); ++u) breg[u] = breg[u + 1];
+            breg[REG ? 15 : 0] = b0;
         }
         gm_sync();
         if (singular) {
@@ -932,16 +912,74 @@ struct SolverT {
         is += gm_shfl_xor(is, 2);
         if (row >= m) is = 0.0;
         const double inorm_inf = block_max(T, [&](int k) { return k == t ? is : 0.0; });
-        const double inorm_1 = block_max(m, [&](int j) {  // column sums are permutation invariant
-            double s = 0;
-            for (int i = 0; i < m; ++i) s += fabs(Bi[i * ldb + j]);
-            return s;
-        });
+        // column sums are permutation invariant
+        const double inorm_1 = block_max(m, [&](int j) { return col_abs_sum(Bi + j, ldb); });
         *cond1 = anorm_1 * inorm_1;
         anorm_w = fmax(anorm_1, anorm_inf);
         const double cond_inf = anorm_inf * inorm_inf;
         cond_inf_last = cond_inf;
         if (!(cond_inf <= GM_CONDITION_TOL)) return 1;
+        return 0;
+    }
+
+    // Elimination step k = 4 jj + kq of invert_basis_reg, with columns 4 jj + q in breg[0] (register slot u holds
+    // columns 4 ((u + jj) mod 16) + q, and prow / t1 entry 4 u + q belongs to that column). Returns 1, before touching
+    // any register, when the pivot is zero or not finite.
+    GM_DEV int eliminate_reg(int k, int kq) {
+        const int t = gm_tid(), T = gm_nthreads();
+        const int row = t >> 2, q = t & 3, lane = t & 31, warp = t >> 5, nw = T >> 5;
+        const bool on_k = q == kq;  // breg[0] of this lane is column k
+        const double sel = breg[0];
+        double key = (on_k && row >= k && row < m) ? fabs(sel) : -1.0;
+        if (key != key) key = INFINITY;
+        // Idamax: first largest |.| in column k at or below the diagonal (dgetf2.go:43-45). The bit
+        // pattern of a non-negative double is monotone, so two unsigned REDUX.MAX give the maximum
+        // and a REDUX.MIN over the rows that hold it gives the first one. key = -1 marks "not a candidate".
+        unsigned long long kb = key >= 0.0 ? gm_d2bits(key) : 0ull;
+        unsigned hi = (unsigned)(kb >> 32), lo = (unsigned)kb;
+        unsigned mh = gm_warp_max_u32(hi);
+        unsigned ml = gm_warp_max_u32(hi == mh ? lo : 0u);
+        int idx = gm_warp_min_int((key >= 0.0 && hi == mh && lo == ml) ? row : INT_MAX);
+        if (lane == 0) { redi[warp] = (int)mh; redi[32 + warp] = (int)ml; redi[64 + warp] = idx; }
+        gm_sync();
+        hi = (unsigned)redi[lane & (nw - 1)];
+        lo = (unsigned)redi[32 + (lane & (nw - 1))];
+        idx = redi[64 + (lane & (nw - 1))];
+        mh = gm_warp_max_u32(hi);
+        ml = gm_warp_max_u32(hi == mh ? lo : 0u);
+        idx = gm_warp_min_int((hi == mh && lo == ml) ? idx : INT_MAX);
+        key = idx == INT_MAX ? -1.0 : gm_bits2d(((unsigned long long)mh << 32) | ml);
+        if (!(key > 0.0) || key == INFINITY) return 1;
+        const int p = idx;
+        double f = gm_shfl_idx(sel, (lane & ~3) | kq);  // my row's entry in column k
+        if (row == p) {
+            const double inv = 1.0 / f;
+#pragma unroll
+            for (int u = 0; u < (REG ? 16 : 1); ++u) prow[4 * u + q] = (u == 0 && on_k ? 1.0 : breg[u]) * inv;
+        }
+        if (row == k && p != k) {
+#pragma unroll
+            for (int u = 0; u < (REG ? 16 : 1); ++u) t1[4 * u + q] = breg[u];
+        }
+        if (t == 0) ipiv[k] = p;
+        gm_sync();
+        if (row == k) {
+#pragma unroll
+            for (int u = 0; u < (REG ? 16 : 1); ++u) breg[u] = prow[4 * u + q];
+        } else {
+            if (row == p) {  // adopt the displaced row k
+#pragma unroll
+                for (int u = 0; u < (REG ? 16 : 1); ++u) breg[u] = t1[4 * u + q];
+                f = t1[kq];  // column k
+            }
+            if (f != 0.0) {
+#pragma unroll
+                for (int u = 0; u < (REG ? 16 : 1); ++u) {
+                    const double base = (u == 0 && on_k) ? 0.0 : breg[u];
+                    breg[u] = base - f * prow[4 * u + q];
+                }
+            }
+        }
         return 0;
     }
 
@@ -2660,8 +2698,12 @@ struct SolverT {
             build_w(n, false);
             invert_basis(&cond1);  // a singular result falls into Phase I like initializeFromBasic's error does
         }
-        recompute_xb_y();
-        if (xb_feasible()) return GM_OK;
+        // y is needed only when this basis is feasible: Phase I recomputes it for its own basis
+        bi_mul(xb, bv);
+        if (xb_feasible()) {
+            bi_mul_t(y, cb);
+            return GM_OK;
+        }
 
         // Phase I (:529-556)
         used_p1 = 1;
@@ -2680,16 +2722,17 @@ struct SolverT {
         if (t == 0) basic[j] = n;
         gm_sync();
         build_w(n + 1, true);
-        recompute_xb_y();
+        bi_mul(xb, bv);
         fresh = false;
         if (!xb_feasible()) {
             double c1;
             const int sing = invert_basis(&c1);
             if (sing) return GM_PANIC_INITIAL_BASIC;  // simplex.go:155-158
-            recompute_xb_y();
+            bi_mul(xb, bv);
             if (!xb_feasible()) return GM_PANIC_INITIAL_BASIC;
             fresh = true;
         }
+        bi_mul_t(y, cb);
         pmark(10, tp);
         int rc = main_loop(GM_PHASE1_TOL, 1, fresh);
         if constexpr (COOP) tp = gm_clock();
